@@ -250,6 +250,46 @@ def md5(b):
     return hashlib.md5(b).hexdigest()
 
 
+# ---------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_LIMIT = 64 << 20
+
+
+class OutputDump:
+    """What the timed path returned in its last step, as DIR/<name>.npy (float32 / float64), so that two builds run with the
+    same arguments (hence the same inputs) can be compared output for output.  Byte strings (coded streams, files) are
+    kept whole for a fixed, seeded sample of them; all files together stay under DUMP_LIMIT bytes."""
+
+    def __init__(self, directory):
+        self.dir = directory
+        self.arrays = {}
+
+    def add(self, name, values, dtype="float64"):
+        import numpy as np
+        self.arrays[name] = np.asarray(values, dtype=dtype)
+
+    def add_bytes(self, name, lengths, fetch, budget):
+        """Byte strings of the given lengths, `fetch(indices)` -> their bytes.  <name>_lengths: every length;
+        <name>_index: a seeded sample of whole strings that fits `budget` bytes as float32; <name>: their bytes, in order."""
+        import numpy as np
+        keep, used = [], 0
+        for i in np.random.default_rng(0).permutation(len(lengths)):
+            if used + 4 * lengths[i] <= budget:
+                keep.append(int(i))
+                used += 4 * lengths[i]
+        keep.sort()
+        self.add(name + "_lengths", lengths)
+        self.add(name + "_index", keep)
+        self.add(name, np.frombuffer(b"".join(fetch(keep)), np.uint8), "float32")
+
+    def write(self):
+        import numpy as np
+        total = sum(a.nbytes + 256 for a in self.arrays.values())          # 256: more than a .npy header takes
+        assert total <= DUMP_LIMIT, "output dump of %d bytes exceeds %d" % (total, DUMP_LIMIT)
+        os.makedirs(self.dir, exist_ok=True)
+        for name, a in self.arrays.items():
+            np.save(os.path.join(self.dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- main
 def main():
     ap = argparse.ArgumentParser()
@@ -260,7 +300,7 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4, 5])
     ap.add_argument("--images", type=int, default=0, help="images per GPU per step (0 = the config's share per GPU)")
     ap.add_argument("--distinct", type=int, default=0, help="distinct synthetic images replicated to --images (0 = per config)")
-    ap.add_argument("--e2e-steps", type=int, default=5)
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the file-level legs (0 = --steps)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-only", action="store_true", help="diagnostic: skip the device-resident legs (the line then has no `value`)")
     ap.add_argument("--no-decode", action="store_true")
@@ -269,8 +309,11 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=512)
     ap.add_argument("--batch", type=int, default=1024, help="config 5: files per decode call (latency = time of a call)")
     ap.add_argument("--streams", type=int, default=4, help="config 5: decode calls in flight (one codec + one submitting thread each), like a server that keeps several requests going")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed legs returned in their last step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     cfg = args.config
+    if args.e2e_steps <= 0:
+        args.e2e_steps = args.steps
     if args.images <= 0:
         args.images = DEFAULT_IMAGES[cfg]
     if args.distinct <= 0:
@@ -381,6 +424,7 @@ def main():
     line = {"metric": metric, "unit": "MB/s", "n_gpus": max(world, 1), "steps": args.steps, "warmup": args.warmup,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "int16 coefficients / u8 probabilities (integer)", "data": "synthetic", "config": config}
+    dump = OutputDump(args.dump_outputs) if args.dump_outputs and rank == 0 else None
 
     # ================================================================== device-resident legs (config 2 only)
     sampler = ClockSampler(local_rank)
@@ -433,6 +477,11 @@ def main():
         # ---------------------------------------------------------------- decode direction + round trip (same batch)
         res = codec.encode_fetch(copy=True)                       # streams of the last launch, on the host
         streams = [[s.data for s in r] for r in res]
+        if dump:
+            segs = [s for r in res for s in r]
+            dump.add("encode_status", [s.status for s in segs])
+            dump.add("encode_ndecisions", [s.ndecisions for s in segs])
+            dump.add_bytes("encode_streams", [len(s.data) for s in segs], lambda ix: [segs[i].data for i in ix], 16 << 20)
         from lepton_b200 import CoefImage
         outs = [CoefImage(ncmp=im.ncmp, mcuv=im.mcuv, bch=im.bch, bcv=im.bcv, qtables_zigzag=im.qtables_zigzag,
                           planes=[np.full_like(p, 1) for p in im.planes], luma_y_start=im.luma_y_start) for im in base_imgs]
@@ -457,6 +506,20 @@ def main():
         barrier()
         launches += codec.kernel_launches - l0
         clocks = sampler.stop()
+        if dump:
+            # planes of a seeded sample of 4 images, and of those a seeded sample of blocks: (image, block index over the
+            # image's components in order) -> 64 coefficients
+            pick = sorted(int(i) for i in np.random.default_rng(0).choice(len(imgs), size=min(4, len(imgs)), replace=False))
+            into = {i: [np.empty_like(p) for p in imgs[i].planes] for i in pick}
+            dump.add("decode_status", codec.decode_fetch(into))
+            rows, index = [], []
+            for i in pick:
+                allb = np.concatenate([p.reshape(-1, 64) for p in into[i]])
+                sel = np.sort(np.random.default_rng(i).choice(len(allb), size=min(4096, len(allb)), replace=False))
+                rows.append(allb[sel])
+                index += [(i, int(b)) for b in sel]
+            dump.add("decode_blocks", np.concatenate(rows), "float32")
+            dump.add("decode_block_index", index)
         dec_s = rmax(sum(dms) / 1e3)
         avg_d_s = (sum(dms) / len(dms)) / 1e3
         dmode = int(os.environ.get("LEPB200_DEC_MODE", "0"))
@@ -511,22 +574,28 @@ def main():
             lat = []
             l0 = sum(cdc.kernel_launches for cdc in codecs)
             import queue
+            # a step is one pass over the calls; every pass has its own result arrays, so that no two calls in flight
+            # write to the same one
+            passes = [handles] + [[fc.prepare(leps[i:i + nb]) for i in range(0, args.images, nb)] for _ in range(args.steps - 1)]
             q = queue.Queue()
-            for h in handles:
-                q.put(h)
+            for p in range(args.steps):
+                for h in range(len(handles)):
+                    q.put((p, h))
             lock = threading.Lock()
+            last_call = {}
 
             def serve(cdc):
                 while True:
                     try:
-                        h = q.get_nowait()
+                        p, h = q.get_nowait()
                     except queue.Empty:
                         return
                     t1 = time.perf_counter()
-                    cdc.decompress(h, copy=False)
+                    cdc.decompress(passes[p][h], copy=False)
                     d1 = time.perf_counter() - t1
                     with lock:
                         lat.append(d1)
+                    last_call[id(cdc)] = (p, h)
             t0 = time.perf_counter()
             ths = [threading.Thread(target=serve, args=(cdc,)) for cdc in codecs]
             for t in ths:
@@ -536,13 +605,22 @@ def main():
             barrier()
             dt = rmax(time.perf_counter() - t0)
             nlaunch = sum(cdc.kernel_launches for cdc in codecs) - l0
+            if dump:
+                # the last call of every codec still holds its output: of those in the last pass, file h * nb + k of call h
+                last = passes[-1]
+                files = [(h, k) for p, h in sorted(last_call.values()) if p == args.steps - 1 for k in range(last[h][1])]
+                got = [fc.results(last[h], [k], copy=False)[0] for h, k in files]
+                dump.add("decompress_files", [h * nb + k for h, k in files])
+                dump.add("decompress_status", [st for st, _ in got])
+                dump.add_bytes("decompress_jpeg", [n for _, n in got],
+                               lambda ix: [fc.results(last[files[i][0]], [files[i][1]])[0][1] for i in ix], 48 << 20)
             for cdc in codecs[1:]:
                 cdc.close()
             lat.sort()
             total_jpeg = rsum(jpeg_bytes)
-            v = total_jpeg / dt / 1e6
-            line.update(value=v, ms_per_step=1e3 * dt, clocks=sampler.stop(), gpu_launches=int(nlaunch),
-                        images_per_s=rsum(args.images) / dt,
+            v = total_jpeg * args.steps / dt / 1e6
+            line.update(value=v, ms_per_step=1e3 * dt / args.steps, clocks=sampler.stop(), gpu_launches=int(nlaunch),
+                        images_per_s=rsum(args.images) * args.steps / dt,
                         latency={"p50_ms": 1e3 * lat[len(lat) // 2], "p90_ms": 1e3 * lat[(len(lat) * 9) // 10], "max_ms": 1e3 * lat[-1],
                                  "files_per_call": nb, "calls": len(lat), "calls_in_flight": K,
                                  "note": "per-image latency = latency of the call that carries the image (one serial chain per thumbnail)"},
@@ -561,9 +639,12 @@ def main():
             l0 = fc.kernel_launches
             t0 = time.perf_counter()
             for _ in range(args.e2e_steps):
-                fc.compress(handle, copy=False)
+                last = fc.compress(handle, copy=False)
             barrier()
             e_s = rmax(time.perf_counter() - t0)
+            if dump:
+                dump.add("compress_status", [st for st, _ in last])
+                dump.add_bytes("compress_lep", [n for _, n in last], lambda ix: [b for _, b in fc.results(handle, ix)], 16 << 20)
             total_jpeg = rsum(jpeg_bytes)
             e2e = {"unit": "MB/s", "h2d_bytes_per_step": int(jpeg_bytes), "d2h_bytes_per_step": int(lep_bytes),
                    "h2d_note": "entropy-coded scan bytes (Huffman decode happens on the GPU); files the host has to decode upload 128 B per block instead",
@@ -580,9 +661,12 @@ def main():
                 l0 = fc.kernel_launches
                 t0 = time.perf_counter()
                 for _ in range(args.e2e_steps):
-                    fc.decompress(lhandle, copy=False)
+                    last = fc.decompress(lhandle, copy=False)
                 barrier()
                 d_s = rmax(time.perf_counter() - t0)
+                if dump:
+                    dump.add("decompress_status", [st for st, _ in last])
+                    dump.add_bytes("decompress_jpeg", [n for _, n in last], lambda ix: [b for _, b in fc.results(lhandle, ix)], 16 << 20)
                 e2e["gpu_launches"] += fc.kernel_launches - l0
                 e2e["d2h_bytes_per_step"] += int(jpeg_bytes)
                 e2e["h2d_bytes_per_step"] += int(lep_bytes)
@@ -628,6 +712,8 @@ def main():
         for k in ("value", "e2e"):
             line.pop(k, None)
         rc = 3
+    if dump:
+        dump.write()
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

@@ -252,10 +252,22 @@ class LeptonB200Codec:
     def decode_launch(self):
         self._check(self._L.lepb200_decode_launch(self._ctx), "decode_launch")
 
-    def decode_fetch(self):
+    def decode_fetch(self, into=None):
+        """Copies the planes of the last decode_launch into the uploaded images' planes and returns per-segment status
+        codes.  ``into`` ({image index: list of per-component int16 arrays}) copies only those images, into those arrays."""
         n = sum(im.nseg for im in self._dec_imgs)
         st = (ctypes.c_int32 * n)()
-        self._check(self._L.lepb200_decode_fetch(self._ctx, self._dec_c, len(self._dec_imgs), st), "decode_fetch")
+        dst = self._dec_c
+        if into is not None:
+            dst = (_Image * len(self._dec_imgs))()
+            for i in range(len(self._dec_imgs)):
+                dst[i] = self._dec_c[i]
+                for c in range(dst[i].ncmp):
+                    p = into.get(i)
+                    if p is not None and (p[c].dtype != np.int16 or not p[c].flags["C_CONTIGUOUS"] or p[c].size != dst[i].bch[c] * dst[i].bcv[c] * 64):
+                        raise LeptonB200Error("plane %d of image %d must be C-contiguous int16 of bch*bcv*64 elements" % (c, i))
+                    dst[i].planes[c] = p[c].ctypes.data if p is not None else None
+        self._check(self._L.lepb200_decode_fetch(self._ctx, dst, len(self._dec_imgs), st), "decode_fetch")
         return list(st)
 
     def decode_images(self, images, streams):
@@ -555,6 +567,16 @@ class LeptonB200FileCodec:
         if not copy:
             return [(res[i].status, res[i].len) for i in range(n)]
         return [(res[i].status, ctypes.string_at(res[i].data, res[i].len) if res[i].len else b"") for i in range(n)]
+
+    @staticmethod
+    def results(handle, indices, copy: bool = True):
+        """(status, bytes) of files ``indices`` of the last compress / decompress call made with a prepare() handle, also
+        after copy=False (with copy=False: (status, length)).  The bytes belong to the codec that made them and are valid
+        until its next call."""
+        res = handle[3]
+        if not copy:
+            return [(res[i].status, res[i].len) for i in indices]
+        return [(res[i].status, ctypes.string_at(res[i].data, res[i].len) if res[i].len else b"") for i in indices]
 
     @property
     def last_gpu_recoded(self):

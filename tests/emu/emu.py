@@ -36,8 +36,11 @@ def build(out=OUT, defines=()):
     if os.path.exists(out) and all(os.path.getmtime(out) >= os.path.getmtime(s) for s in SOURCES):
         return out
     os.makedirs(os.path.dirname(out), exist_ok=True)
+    # compile to a private name and rename: parallel test workers may build at once, and none may load a half-written file
+    tmp = "%s.%d.tmp" % (out, os.getpid())
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++", "-I", os.path.join(HERE, "fake"),
-                           "-Wno-unknown-pragmas"] + ["-D" + d for d in defines] + ["-o", out, os.path.join(HERE, "emu_kernels.cc")])
+                           "-Wno-unknown-pragmas"] + ["-D" + d for d in defines] + ["-o", tmp, os.path.join(HERE, "emu_kernels.cc")])
+    os.replace(tmp, out)
     return out
 
 

@@ -98,3 +98,50 @@ def oracle_encode_image(img):
         y1 = img.bcv[0] if last else starts[i + 1]
         out.append(oracle.encode_segment(g, img.planes, y0, y1, last))
     return out
+
+
+def synth_jpeg(w, h, quality, subsampling, progressive=False, seed=0):
+    """A photo-sized JPEG generated on the spot (stands in for test images too large to keep in the repository).  The
+    pixels come from integer arithmetic only, so they are the same on every machine; Pillow's libjpeg writes the file."""
+    import io
+    from PIL import Image, ImageFile
+    ImageFile.MAXBLOCK = 1 << 26
+    rng = np.random.default_rng(seed)
+    img = np.full((h, w, 3), 96, np.int32)
+    for scale, amp in ((256, 96), (64, 48), (16, 24), (4, 12), (1, 6)):
+        n = rng.integers(0, amp, (h // scale + 1, w // scale + 1, 3), dtype=np.int32)
+        img += np.repeat(np.repeat(n, scale, 0), scale, 1)[:h, :w]
+    b = io.BytesIO()
+    Image.fromarray(np.clip(img - 93, 0, 255).astype(np.uint8), "RGB").save(
+        b, "JPEG", quality=quality, subsampling=subsampling, progressive=progressive, optimize=False)
+    return b.getvalue()
+
+
+def mixed_corpus_jpegs():
+    """36 small JPEGs of mixed size (incl. odd sizes), chroma subsampling, quality, with and without restart markers, some
+    progressive, some grey (BASELINE config 3 in miniature)."""
+    import io
+    from PIL import Image, ImageFile
+    ImageFile.MAXBLOCK = 1 << 24
+    rng = np.random.default_rng(20240917)
+    jpegs = []
+    for k in range(36):
+        w, h = int(rng.integers(9, 700)), int(rng.integers(9, 500))
+        y, x = np.mgrid[0:h, 0:w]
+        base = (128 + 70 * np.sin(x / (5.0 + k)) + 50 * np.cos(y / (3.0 + 0.5 * k)))[..., None] + rng.normal(0, 6 + 3 * (k % 7), (h, w, 3))
+        im = Image.fromarray(np.clip(base, 0, 255).astype(np.uint8))
+        kw = dict(quality=[60, 75, 85, 95, 100][k % 5])
+        if k % 9 == 8:
+            im = im.convert("L")
+        else:
+            kw["subsampling"] = k % 3
+        if k % 4 == 3:
+            kw["restart_marker_blocks"] = 1 + k % 5
+        if k % 6 == 5:
+            kw["progressive"] = True
+        if k % 10 == 7:
+            kw["optimize"] = True
+        b = io.BytesIO()
+        im.save(b, "JPEG", **kw)
+        jpegs.append(b.getvalue())
+    return jpegs

@@ -269,26 +269,30 @@ def test_minencodethreads_reproduces_reference_containers(lep_name, min_threads)
     assert hj.write_lep(lepfmt.demux(lf.payload)[:lf.nseg]) == ref
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/images"), reason="reference tree only exists in the build container")
 @pytest.mark.parametrize("flags", [["-maxencodethreads=1"], ["-maxencodethreads=2"], ["-maxencodethreads=3", "-minencodethreads=3"],
                                    ["-minencodethreads=8"], ["-minencodethreads=5", "-maxencodethreads=6"],
                                    ["-evensplit"], ["-evensplit", "-minencodethreads=8"]])
-def test_encode_thread_flags_against_live_reference(flags, tmp_path):
-    """Splits chosen under -minencodethreads / -maxencodethreads / -evensplit == the unmodified reference CLI's, on files of three sizes."""
-    import subprocess
-    from conftest import REF_LEPTON
+def test_encode_thread_flags_against_live_reference(flags):
+    """Splits chosen under -minencodethreads / -maxencodethreads / -evensplit == the unmodified reference CLI's, on files of
+    three sizes (the largest a 24 MP tests/helpers.synth_jpeg one); the container around the oracle's streams for those
+    splits == the reference's file (md5).  The reference's results: tests/golden/reference_cpu.json."""
+    import hashlib
+    import json
+    from helpers import oracle_encode_image, synth_jpeg
     from lepton_b200 import HostJpeg
+    ref = json.load(open(os.path.join(GOLDEN, "reference_cpu.json")))["thread_flags"][" ".join(flags)]
     lo = max([int(f.split("=")[1]) for f in flags if f.startswith("-min")] + [1])
     hi = min([int(f.split("=")[1]) for f in flags if f.startswith("-max")] + [8])
-    for name in ("iphonecrop.jpg", "androidcrop.jpg", "slrcity.jpg"):
-        jpg = os.path.join("/root/reference/images", name)
-        lep = str(tmp_path / (name + ".lep"))
-        assert subprocess.run([REF_LEPTON, "-skipverify", "-unjailed"] + flags + [jpg, lep], capture_output=True).returncode == 0
-        lf = lepfmt.parse_container(open(lep, "rb").read())
-        hj = HostJpeg(open(jpg, "rb").read(), min_threads=lo, max_threads=hi, even_split="-evensplit" in flags)
+    assert sorted(ref) == ["androidcrop.jpg", "iphonecrop2.jpg", "synth_6000x4000_q95_444.jpg"]
+    for name, want in sorted(ref.items()):
+        jpg = open(os.path.join(GOLDEN, want["fixture"]), "rb").read() if "fixture" in want else synth_jpeg(**want["synth"])
+        hj = HostJpeg(jpg, min_threads=lo, max_threads=hi, even_split="-evensplit" in flags)
         assert hj.status == 0, hj.error
-        assert list(hj.coef_image().luma_y_start) == [h.luma_y_start for h in lf.handoffs], (name, flags)
-        assert hj.write_lep(lepfmt.demux(lf.payload)[:lf.nseg]) == open(lep, "rb").read(), (name, flags)
+        img = hj.coef_image()
+        assert list(img.luma_y_start) == want["luma_y_start"], (name, flags)
+        enc = oracle_encode_image(img)
+        assert [rc for rc, _, _ in enc] == [0] * len(enc), (name, flags)
+        assert hashlib.md5(hj.write_lep([s for _, s, _ in enc])).hexdigest() == want["lep_md5"], (name, flags)
 
 
 def test_roundtripfail_fixture_host_halves():
